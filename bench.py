@@ -2,7 +2,7 @@
 """bench.py -- headline benchmark of the streaming hot path (BASELINE.json metric: RTFx = audio seconds
 processed per wall second, summed over streams; per-chunk latency alongside).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config C] [--only-headline]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config C] [--only-headline] [--dump-outputs DIR]
 
 Headline (top-level keys of the JSON line) = BASELINE.json configs[1] ("config 2"): nemotron-speech-streaming-en-0.6b
 (24 layers, random-init synthetic weights of that architecture), bf16 compute, 64 concurrent streams per GPU, 160 ms chunks
@@ -25,6 +25,10 @@ Per config:
   latency : host-to-host, one chunk at a time as a real-time feed sees it: clock starts when the chunk's last sample is handed to
             nsb_push_pcm_batch and stops when its token ids are back on the host (graph-capture step excluded)
   roofline: the dominant kernel class (tcgen05 layer GEMMs) timed alone, live, against MEASURED_PEAKS.json
+
+--dump-outputs DIR writes, for the headline config, what its last timed step computed: encoder_out.npy = the encoder output of the
+last device-resident step [streams x (1 + R), 1024], tokens.npy = the token ids the last e2e step handed back [streams, 12 (1 + R)],
+-1 past each stream's count. The inputs are seeded, so two builds run with the same arguments can be compared array for array.
 
 --impl reference times the CPU oracle port of the reference path (oracle/liboracle.so, all host threads): every step = one chunk
 of a bounded number of streams, `ms_per_step` is its measured wall time. The reference's own ggml build cannot be produced
@@ -244,6 +248,24 @@ def run_reference(args, rank: int):
     print(json.dumps(line), flush=True)
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def write_dump(d: str, arrays: dict) -> None:
+    """--dump-outputs: each array as DIR/<name>.npy in float32. An array whose share of the 64 MB limit is too small keeps a fixed,
+    seeded sample of its rows, and DIR/<name>_rows.npy (float64) says which."""
+    os.makedirs(d, exist_ok=True)
+    share = DUMP_LIMIT // len(arrays)
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float32)
+        if a.nbytes > share:
+            keep = share // (a[0].nbytes + 8)                # + its float64 row index
+            rows = np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))
+            np.save(os.path.join(d, f"{name}_rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(d, f"{name}.npy"), a)
+
+
 def token_checksum(per_stream):
     """Order-sensitive checksum of {global stream id: token list}."""
     c = 0
@@ -271,7 +293,7 @@ def run_config(no: int, args, ctx, headline: bool):
         total = max(1, total // int(os.environ["NSB_BENCH_EMULATE_WORLD"]))
     mine = sharding.local_streams(range(total), rank, world)
     S = len(mine)
-    steps = args.steps if headline else max(5, min(args.steps, int(os.environ.get("NSB_BENCH_SIDE_STEPS", 20))))
+    steps = args.steps
     warm_chunks = 40 if no == 2 else max(8, 70 // T + 3)          # > 70 / T: the attention cache is full (steady state) before timing
     hbm_peak, tf_peak, peak_kind = peaks()
 
@@ -315,6 +337,9 @@ def run_config(no: int, args, ctx, headline: bool):
     sync_all()
     wall = time.perf_counter() - t0
     clocks = sampler.stop()
+    dump = {}
+    if headline and args.dump_outputs and rank == 0:
+        dump["encoder_out"] = eng.debug_get("x", S)       # the last timed step's encoder output, before anything else runs
     launches = int(eng.stats().kernel_launches - st0.kernel_launches)
     dev_lat = sorted(eng.bench_step() for _ in range(min(steps, 30)))     # device time of single host-synchronised steps
     t_dev_s, wall_s = max_over_ranks(dev_ms / 1e3, wall)
@@ -362,15 +387,18 @@ def run_config(no: int, args, ctx, headline: bool):
     ids = np.arange(S, dtype=np.int32)
     pos = 0
     toks = {g: [] for g in mine}
+    popped = None
 
     def feed(n):
         nonlocal pos
         eng.push_batch(ids, pcm2[:, pos:pos + n]); pos += n
 
     def pop():
+        nonlocal popped
         out, cnt = eng.pop_tokens_batch(ids, 12 * T)
         for i, g in enumerate(mine):
             toks[g] += out[i, :cnt[i]].tolist()
+        popped = (out, cnt)
         return int(cnt.sum())
 
     feed(first)
@@ -396,6 +424,10 @@ def run_config(no: int, args, ctx, headline: bool):
     sync_all()
     e2e_wall = time.perf_counter() - t0
     (t_e2e,) = max_over_ranks(e2e_wall)
+    if dump:
+        out, cnt = popped                                  # token ids of the last timed step, per stream, -1 past each count
+        dump["tokens"] = np.where(np.arange(out.shape[1]) < cnt[:, None], out, -1)
+        write_dump(args.dump_outputs, dump)
     # ---- host-to-host chunk latency: one chunk at a time, as a real-time feed sees it ----
     lat = []
     for _ in range(n_lat):
@@ -456,6 +488,7 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--config", type=int, default=2, choices=sorted(CONFIGS), help="BASELINE.json config in the headline keys (default 2)")
     ap.add_argument("--only-headline", action="store_true", help="skip the `configs` record (the other BASELINE.json configs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the headline config's last timed step computed to DIR/*.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", 0)); world = int(os.environ.get("WORLD_SIZE", 1)); local = int(os.environ.get("LOCAL_RANK", 0))
     if args.impl == "reference":

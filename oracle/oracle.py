@@ -10,6 +10,9 @@ import subprocess
 import numpy as np
 
 _DIR = os.path.dirname(os.path.abspath(__file__))
+# Optional checkout of the reference project (nemotron-speech.cpp). Only the differential tests that compile or run the reference's
+# own sources use it; they skip without it, and the committed fixtures under tests/golden/ stand in for it.
+REFERENCE_DIR = os.environ.get("NSB_REFERENCE_DIR", "")
 MM_REF, MM_F16, MM_BF16, MM_Q8FAST = 0, 1, 2, 3
 KV_F32, KV_F16, KV_BF16 = 0, 1, 2
 
@@ -18,11 +21,17 @@ _i16p = np.ctypeslib.ndpointer(dtype=np.int16, flags="C_CONTIGUOUS")
 _i32p = np.ctypeslib.ndpointer(dtype=np.int32, flags="C_CONTIGUOUS")
 
 
+def reference_file(rel: str) -> str | None:
+    """Path of `rel` inside the reference checkout, or None when there is no checkout or it lacks the file."""
+    p = os.path.join(REFERENCE_DIR, rel) if REFERENCE_DIR else ""
+    return p if p and os.path.exists(p) else None
+
+
 def build(force: bool = False) -> None:
     so = os.path.join(_DIR, "liboracle.so")
     src = os.path.join(_DIR, "stream_oracle.cpp")
     stale = (not os.path.exists(so)) or os.path.getmtime(so) < os.path.getmtime(src)
-    if force or stale or (os.path.isdir("/root/reference/src") and not os.path.exists(os.path.join(_DIR, "_ref", "libnemo_ref.so"))):
+    if force or stale or (reference_file("src") and not os.path.exists(os.path.join(_DIR, "_ref", "libnemo_ref.so"))):
         subprocess.check_call(["make", "-C", _DIR, "all"], stdout=subprocess.DEVNULL)
 
 

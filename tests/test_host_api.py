@@ -8,6 +8,7 @@ import subprocess
 import numpy as np
 import pytest
 
+import oracle as O
 import synth
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -84,13 +85,13 @@ def test_product_sources_do_not_touch_the_oracle():
         assert "liboracle" not in open(os.path.join(ROOT, f)).read()
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/src/transcribe_stream.cpp"), reason="reference sources not present")
+@pytest.mark.skipif(not O.reference_file("src/transcribe_stream.cpp"), reason="no reference checkout (NSB_REFERENCE_DIR)")
 def test_reference_cli_compiles_unmodified_against_dropin_headers(built, tmp_path):
     exe = tmp_path / "nemotron-asr"
     pkg = os.path.join(ROOT, "nemotron-speech.cpp_b200")
     # a quoted #include looks next to the source file first, so build a byte-identical copy outside the reference tree
     src = tmp_path / "transcribe_stream.cpp"
-    src.write_bytes(open("/root/reference/src/transcribe_stream.cpp", "rb").read())
+    src.write_bytes(open(O.reference_file("src/transcribe_stream.cpp"), "rb").read())
     cmd = ["/usr/bin/g++", "-std=c++17", "-O2", "-I", os.path.join(ROOT, "include"), str(src),
            "-L", pkg, "-lnsb200", f"-Wl,-rpath,{pkg}", "-o", str(exe)]
     subprocess.check_call(cmd)
@@ -100,7 +101,7 @@ def test_reference_cli_compiles_unmodified_against_dropin_headers(built, tmp_pat
     assert r.returncode == 1 and "Failed to load model" in r.stderr          # :102-105
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/src/transcribe.cpp"), reason="reference sources not present")
+@pytest.mark.skipif(not O.reference_file("src/transcribe.cpp"), reason="no reference checkout (NSB_REFERENCE_DIR)")
 def test_reference_batch_cli_compiles_unmodified_against_dropin_headers(built, tmp_path):
     """src/transcribe.cpp (the non-streaming CLI) against include/: nemo_transcribe_audio exists in the shim (its CUDA side is
     experimental this round); usage and load-failure behaviour are the reference's (transcribe.cpp:31-34,52-56)."""
@@ -113,7 +114,7 @@ def test_reference_batch_cli_compiles_unmodified_against_dropin_headers(built, t
     for h in os.listdir(os.path.join(ROOT, "include")):
         shutil.copy(os.path.join(ROOT, "include", h), tmp_path / "src" / h)
     src = tmp_path / "src" / "transcribe.cpp"
-    src.write_bytes(open("/root/reference/src/transcribe.cpp", "rb").read())
+    src.write_bytes(open(O.reference_file("src/transcribe.cpp"), "rb").read())
     subprocess.check_call(["/usr/bin/g++", "-std=c++17", "-O2", "-I", os.path.join(ROOT, "include"), str(src),
                            "-L", pkg, "-lnsb200", f"-Wl,-rpath,{pkg}", "-o", str(exe)])
     r = subprocess.run([str(exe)], capture_output=True, text=True)
@@ -160,26 +161,31 @@ typedef struct ggml_backend* ggml_backend_t; typedef struct ggml_backend_buffer*
 """
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/src/nemo-stream.h"), reason="reference sources not present")
 def test_dropin_headers_agree_with_the_reference_headers(tmp_path):
     """Differential test of the host-side logic that lives in the headers (what the reference's tests/test_streaming.cpp unit
     tests poke: chunk / shift / latency arithmetic of every latency mode and factory, nemo_decoder_state init / reset,
-    timed_token::to_seconds, hparams defaults, enum values): the same probe is compiled once against the REFERENCE's own
-    src/nemo-stream.h + src/nemo-ggml.h (ggml's headers replaced by empty forward-declaration stubs; header-only, nothing of the
-    reference is linked) and once against include/, and must print the same."""
+    timed_token::to_seconds, hparams defaults, enum values): the probe compiled against include/ must print what it printed
+    compiled against the REFERENCE's own src/nemo-stream.h + src/nemo-ggml.h (ggml's headers replaced by empty forward-declaration
+    stubs; header-only, nothing of the reference is linked). That output is committed (tests/golden/header_probe_ref.txt); with a
+    reference checkout the probe is also compiled against its headers again."""
     stub = tmp_path / "stub"; stub.mkdir()
     (stub / "ggml.h").write_text(GGML_STUB)
     for h in ("ggml-cpu.h", "ggml-alloc.h", "ggml-backend.h", "gguf.h"):
         (stub / h).write_text("#pragma once\n")
     src = tmp_path / "probe.cpp"
     src.write_text(HEADER_PROBE)
-    outs = []
-    for name, incs in (("ref", [str(stub), "/root/reference/src"]), ("ours", [os.path.join(ROOT, "include")])):
+    with open(os.path.join(ROOT, "tests", "golden", "header_probe_ref.txt")) as f:
+        outs = [f.read()]
+    builds = [("ours", [os.path.join(ROOT, "include")])]
+    if O.reference_file("src/nemo-stream.h"):
+        builds.append(("ref", [str(stub), O.reference_file("src")]))
+    for name, incs in builds:
         exe = tmp_path / f"probe_{name}"
         cmd = ["/usr/bin/g++", "-std=c++17", "-O1"] + [f"-I{i}" for i in incs] + [str(src), "-o", str(exe)]
         subprocess.check_call(cmd)
         outs.append(subprocess.check_output([str(exe)], text=True))
-    assert outs[0] == outs[1], "\n--- reference headers\n" + outs[0] + "--- drop-in headers\n" + outs[1]
+    for out in outs[1:]:
+        assert out == outs[0], "\n--- reference headers\n" + outs[0] + "--- this build\n" + out
     assert "chunk_mel=121" in outs[1] and "samples=19360" in outs[1] and "latency_ms=1210" in outs[1]      # R = 13 (SURVEY appendix B)
 
 

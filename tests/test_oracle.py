@@ -70,7 +70,7 @@ def test_model_math_matches_reference_golden(built, model2):
     assert np.array_equal(s.tokens(), g["tokens"])                    # greedy: exact token match (test_compute.cpp:2808-2820)
 
 
-@pytest.mark.skipif(not O.ref_available(), reason="oracle/_ref/libnemo_ref.so not built (needs /root/reference)")
+@pytest.mark.skipif(not O.ref_available(), reason="oracle/_ref/libnemo_ref.so not built (needs a reference checkout, NSB_REFERENCE_DIR)")
 def test_against_compiled_reference_all_latency_modes(built, model2):
     fb, win = synth.mel_filterbank(), synth.gen_tensor("w", (400,), ("window", 0), 1234, 0, 0)
     pcm = synth.synth_pcm(5, 1.5)
@@ -116,7 +116,7 @@ def _cached_stream_from_reference_modules(model2, rw, R, secs):
     return n_chunks, worst, rw.greedy(np.concatenate(encs)), s.tokens()
 
 
-@pytest.mark.skipif(not O.ref_available(), reason="oracle/_ref/libnemo_ref.so not built (needs /root/reference)")
+@pytest.mark.skipif(not O.ref_available(), reason="oracle/_ref/libnemo_ref.so not built (needs a reference checkout, NSB_REFERENCE_DIR)")
 def test_cached_streaming_steps_match_reference_modules_past_the_cache_roll(built, model2):
     """Pins the CACHED step (K/V cache + mask + rel-shift over K = 70 + T keys, conv cache, cache roll once more than 70 frames
     went by, decoder state carried across chunks) -- the part no runnable reference test covers -- against the reference's own
@@ -137,7 +137,7 @@ def test_cached_streaming_steps_match_reference_modules_past_the_cache_roll(buil
 @pytest.mark.parametrize("R,secs", [(0, 6.0), (1, 6.6), (6, 7.5), (13, 9.0)])
 def test_cached_streaming_matches_reference_golden(built, model2, R, secs):
     """The committed fixture of the test above (tests/golden/cached_ref_L2.npz, tools/make_golden.py section 3): holds where
-    /root/reference is absent. All tokens of the stream + the encoder output of the last chunk (cache rolled)."""
+    no reference checkout is available. All tokens of the stream + the encoder output of the last chunk (cache rolled)."""
     g = np.load(os.path.join(GOLD, "cached_ref_L2.npz"))
     s = O.Stream(model2, R, trace=True)
     s.push(synth.synth_pcm(11, secs))
@@ -147,7 +147,7 @@ def test_cached_streaming_matches_reference_golden(built, model2, R, secs):
     assert np.array_equal(s.tokens(), g[f"tokens_R{R}"])
 
 
-@pytest.mark.skipif(not O.ref_available(), reason="oracle/_ref/libnemo_ref.so not built (needs /root/reference)")
+@pytest.mark.skipif(not O.ref_available(), reason="oracle/_ref/libnemo_ref.so not built (needs a reference checkout, NSB_REFERENCE_DIR)")
 def test_batch_path_matches_compiled_reference(built, model2):
     """SURVEY 8f.1, oracle side only (no CUDA batch path yet): the non-streaming nemo_encode path -- whole-utterance subsampling
     with no carried / dropped frames, non-cached layers, greedy from a fresh decoder state -- against the reference's compiled
@@ -297,7 +297,7 @@ def test_detokeniser(built, model2):
     assert model2.detok(ids) == expect
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/scripts/compare_tensors.py"), reason="reference scripts not present")
+@pytest.mark.skipif(not O.reference_file("scripts/compare_tensors.py"), reason="no reference checkout (NSB_REFERENCE_DIR)")
 def test_encoder_dump_is_readable_by_the_reference_compare_script(built, model2, tmp_path):
     """tools/dump_encoder_out.py writes per-chunk encoder output in the reference's own dump format (nemo-stream.cpp:886-958); the
     reference's scripts/compare_tensors.py must load it (its loader reads the first chunk) and report it identical to itself."""
@@ -309,7 +309,7 @@ def test_encoder_dump_is_readable_by_the_reference_compare_script(built, model2,
     out = tmp_path / "enc.bin"
     tool = os.path.join(os.path.dirname(GOLD), "..", "tools", "dump_encoder_out.py")
     subprocess.check_call([sys.executable, tool, "--impl", "oracle", synth.cached_model("f32", 2, R=0), str(f), "6", str(out)])
-    spec = importlib.util.spec_from_file_location("ref_compare_tensors", "/root/reference/scripts/compare_tensors.py")
+    spec = importlib.util.spec_from_file_location("ref_compare_tensors", O.reference_file("scripts/compare_tensors.py"))
     ref = importlib.util.module_from_spec(spec); spec.loader.exec_module(ref)
     t = ref.load_tensor(str(out))
     s = O.Stream(model2, 6, trace=True); s.push(pcm)

@@ -8,6 +8,7 @@ import subprocess
 import numpy as np
 import pytest
 
+import oracle as O
 import synth
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -219,7 +220,7 @@ def test_serve_realtime_on_the_mock_engine(mock_exe, tmp_path):
     assert 0.8 <= wall <= 1.6                                            # 1 s of audio paced at audio rate
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/src/transcribe_stream.cpp"), reason="reference sources not present")
+@pytest.mark.skipif(not O.reference_file("src/transcribe_stream.cpp"), reason="no reference checkout (NSB_REFERENCE_DIR)")
 @pytest.mark.parametrize("R", [0, 1, 6, 13])
 def test_reference_cli_on_the_shim_and_the_mock_engine(tmp_path, R):
     """The reference's own streaming CLI (byte-identical) + the drop-in shim (csrc/nemo_shim.cpp) + the test double of the C ABI, on
@@ -229,7 +230,7 @@ def test_reference_cli_on_the_shim_and_the_mock_engine(tmp_path, R):
     T = R + 1
     csrc = os.path.join(ROOT, "nemotron-speech.cpp_b200", "csrc")
     src = tmp_path / "transcribe_stream.cpp"
-    src.write_bytes(open("/root/reference/src/transcribe_stream.cpp", "rb").read())
+    src.write_bytes(open(O.reference_file("src/transcribe_stream.cpp"), "rb").read())
     exe = tmp_path / "cli_mock"
     subprocess.check_call(["/usr/bin/g++", "-std=c++17", "-O1", "-I", os.path.join(ROOT, "include"), "-I", csrc, str(src),
                            os.path.join(csrc, "nemo_shim.cpp"), os.path.join(ROOT, "tests", "mock_nsb200.cpp"), "-o", str(exe)])

@@ -22,6 +22,7 @@ import argparse
 import os
 import re
 import struct
+import tempfile
 import zlib
 
 import numpy as np
@@ -458,7 +459,8 @@ def cached_model(kind: str, n_layers: int, seed: int = 1234, cache_dir: str | No
     """Materialise (once) and return the path of a synthetic model file. kind: f32|f16|q8_0|q4_0|nemo.
     R = latency mode whose calibration (tools/calib/) shapes joint.enc.bias and the blank bias;
     profile = "parity" (tests) | "speech" (bench: speech-like token rate, see load_calibration)."""
-    cache_dir = cache_dir or os.environ.get("NSB_SYNTH_DIR", "/tmp/nsb200_synth")
+    # per user: a directory another user created first would not be writable
+    cache_dir = cache_dir or os.environ.get("NSB_SYNTH_DIR") or os.path.join(tempfile.gettempdir(), f"nsb200_synth_{os.getuid()}")
     os.makedirs(cache_dir, exist_ok=True)
     ext = "bin" if kind == "nemo" else "gguf"
     tag = "" if profile == "parity" else f"_{profile}"
