@@ -183,6 +183,41 @@ int nsb_debug_get_cache(nsb_engine* e, int stream, int which /*0=k,1=v,2=conv*/,
 int nsb_op_logmel(nsb_engine* e, const int16_t* pcm, int n_streams, int n_samples, float* mel_out, size_t cap_floats);
 int nsb_op_gemm(nsb_engine* e, const char* weight_name, const float* x, int rows, float* y, size_t cap_floats);
 
+/* ---- operator tests of the step's GEMM and LayerNorm launches (host in / host out) ----------------------------------------
+ * nsb_op_gemm_ex: one GEMM C = epi(x W^T) on a weight nsb_op_gemm takes (per-layer matrices, and the matrices every GGUF keeps in
+ *   F32: encoder.pre_encode.conv.3 / conv.6 / out, joint.enc -- 3xTF32 on the tensor cores; pre_encode.out expects x in the engine's
+ *   (w * 256 + c) column order), launched through the engine's own dispatch with the settings below. x [rows][n_in] f32 is rounded to
+ *   the engine's activation type like the step's producers (F32 matrices: plain f32). The destination (and the split-K workspace) is
+ *   padded with guard rows before and after the live region and 32 unused columns per row (ldc = n_out + 32), all holding a NaN
+ *   pattern; *guard_bad = how many guard elements the GEMM changed (0 = no stray store).
+ *   y receives the raw output bits: [m_out][n_out] elements of out_type (16-bit outputs as stored, 2 bytes each), or for
+ *   NSB_EPI_PARTIAL every k-slice plane [splits][m_out][n_out] f32 (plane 0 from C0 when c0 is set). m_out = rows, or with the
+ *   output row map rows / c_group * (c_group - c_drop). Returns n_out, -bytes needed when y_bytes is too small, <0 on error (a forced
+ *   tile config that is not instantiated for the operand type or whose grid does not cover n_out is NSB_ERR_ARG). */
+enum nsb_epi { NSB_EPI_NONE = 0, NSB_EPI_RELU = 1, NSB_EPI_SILU = 2, NSB_EPI_RESID = 3, NSB_EPI_PARTIAL = 4 };
+enum nsb_out_type { NSB_OUT_F32 = 0, NSB_OUT_F16 = 1, NSB_OUT_BF16 = 2 };
+typedef struct nsb_gemm_op {
+    const char* weight;        /* tensor name                                                                             */
+    int32_t rows;              /* rows of x (M)                                                                           */
+    int32_t epi;               /* enum nsb_epi: NONE / RELU (+bias) / SILU / RESID (C += alpha acc, f32) / PARTIAL (split-K)  */
+    float alpha;               /* NSB_EPI_RESID                                                                           */
+    int32_t out_type;          /* enum nsb_out_type; 16-bit only for NONE / RELU / SILU                                   */
+    int32_t splits;            /* k slices (NSB_EPI_PARTIAL; 1 otherwise)                                                 */
+    int32_t c0;                /* NSB_EPI_PARTIAL: slice 0 (+ bias) goes to its own destination, slices z >= 1 to workspace plane z-1 */
+    int32_t c_group, c_drop;   /* output row map: rows r with r % c_group < c_drop are dropped, the rest compacted (0 = off)  */
+    int32_t force_bn, force_stages;   /* tile config as nsb_bench_gemm takes it; 0 = the engine's own dispatch             */
+    int32_t rotate;            /* CTA n starts its k loop at k-block (n mod nk) (single-CTA tiles)                        */
+    const float* bias;         /* [n_out] or NULL                                                                         */
+    const float* c_init;       /* NSB_EPI_RESID: initial C [m_out][n_out]                                                 */
+} nsb_gemm_op;
+int nsb_op_gemm_ex(nsb_engine* e, const nsb_gemm_op* op, const float* x, void* y, size_t y_bytes, long long* guard_bad);
+/* nsb_op_layernorm: the LayerNorm launch of the step on host rows of 1024: x [rows][1024] f32 += alpha * (sum of n_planes split-K
+ *   planes [n_planes][rows][1024], 0 <= n_planes <= 8, summed in plane order), then fused = 0: y = LN(x; g1, b1) (x keeps the reduced
+ *   rows); fused = 1 (norm_out fused with the next layer's first norm): x = LN(x; g1, b1) and, when g2 is set, y = LN(x; g2, b2).
+ *   eps 1e-5. y: [rows][1024] of out_type; x_out: x after the launch. Returns 0 or <0. */
+int nsb_op_layernorm(nsb_engine* e, const float* x, int rows, const float* planes, int n_planes, float alpha, const float* g1, const float* b1,
+                     const float* g2, const float* b2, int fused, int out_type, float* x_out, void* y);
+
 /* ---- non-streaming batch path: replaces nemo_encode_audio / nemo_transcribe_audio (src/nemo-ggml.cpp:1467-1600) for ONE
  * utterance: whole-utterance log-mel -> subsampling with no carried / dropped frames -> non-cached conformer layers with
  * full-context rel-pos attention -> greedy decode from a fresh decoder state. Validated on hardware against the CPU checker and the

@@ -15,6 +15,8 @@ import numpy as np
 _DIR = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_DIR, "libnsb200.so")
 
+EPI_NONE, EPI_RELU, EPI_SILU, EPI_RESID, EPI_PARTIAL = 0, 1, 2, 3, 4
+OUT_F32, OUT_F16, OUT_BF16 = 0, 1, 2
 COMPUTE_AUTO, COMPUTE_F32, COMPUTE_F16, COMPUTE_BF16, COMPUTE_Q8_0, COMPUTE_Q8_0_STRICT = 0, 1, 2, 3, 4, 5
 KV_F32, KV_F16, KV_BF16 = 0, 1, 2
 
@@ -41,6 +43,12 @@ TRACE_TAGS = {1: "logmel", 2: "stem", 3: "dwconv", 4: "melhist", 5: "gemm_f32", 
               11: "convmod", 12: "advance", 13: "decode", 14: "other"}
 
 
+class GemmOp(C.Structure):
+    _fields_ = [("weight", C.c_char_p), ("rows", C.c_int32), ("epi", C.c_int32), ("alpha", C.c_float), ("out_type", C.c_int32),
+                ("splits", C.c_int32), ("c0", C.c_int32), ("c_group", C.c_int32), ("c_drop", C.c_int32), ("force_bn", C.c_int32),
+                ("force_stages", C.c_int32), ("rotate", C.c_int32), ("bias", C.c_void_p), ("c_init", C.c_void_p)]
+
+
 class ModelInfo(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ("n_mels", "d_model", "n_heads", "d_head", "d_ff", "n_layers", "kernel_size", "vocab_size",
                                          "decoder_dim", "joint_dim", "n_tensors", "weight_type")] + [("vocab", C.c_char * (1025 * 8))]
@@ -51,7 +59,7 @@ EXPORTS = ["nsb_gguf_probe", "nsb_gguf_read_tensor", "nsb_default_config", "nsb_
            "nsb_stream_open", "nsb_stream_close", "nsb_stream_reset", "nsb_stream_push_pcm", "nsb_push_pcm_batch", "nsb_pop_tokens_batch", "nsb_stream_ready", "nsb_engine_step", "nsb_engine_step_begin", "nsb_engine_step_end",
            "nsb_engine_drain", "nsb_stream_pop_tokens", "nsb_stream_chunks", "nsb_detokenize", "nsb_engine_get_stats",
            "nsb_bench_prepare", "nsb_bench_step", "nsb_bench_steps", "nsb_bench_profile", "nsb_profiler_range", "nsb_bench_gemm", "nsb_trace_enable", "nsb_trace_fetch", "nsb_debug_enable", "nsb_debug_get", "nsb_debug_get_cache", "nsb_op_logmel",
-           "nsb_op_gemm", "nsb_transcribe_full"]
+           "nsb_op_gemm", "nsb_op_gemm_ex", "nsb_op_layernorm", "nsb_transcribe_full"]
 
 
 def build(force: bool = False) -> str:
@@ -108,6 +116,8 @@ def lib():
         L.nsb_debug_get_cache.argtypes = [vp, ci, ci, ci, _f32p, C.c_size_t]
         L.nsb_op_logmel.argtypes = [vp, _i16p, ci, ci, _f32p, C.c_size_t]
         L.nsb_op_gemm.argtypes = [vp, C.c_char_p, _f32p, ci, _f32p, C.c_size_t]
+        L.nsb_op_gemm_ex.argtypes = [vp, C.POINTER(GemmOp), _f32p, vp, C.c_size_t, C.POINTER(C.c_longlong)]
+        L.nsb_op_layernorm.argtypes = [vp, _f32p, ci, vp, ci, C.c_float, _f32p, _f32p, vp, vp, ci, ci, _f32p, vp]
         L.nsb_transcribe_full.argtypes = [vp, _i16p, ci, _i32p, _i32p, ci, C.POINTER(C.c_int), C.c_void_p, C.c_size_t]
         _lib = L
     return _lib
@@ -315,6 +325,45 @@ class Engine:
         y = np.empty((x.shape[0], 4096), dtype=np.float32)
         n_out = _check(lib().nsb_op_gemm(self.h, weight_name.encode(), x, x.shape[0], y.reshape(-1), y.size))
         return y.reshape(-1)[: x.shape[0] * n_out].reshape(x.shape[0], n_out).copy()
+
+    def op_gemm_ex(self, weight_name: str, x: np.ndarray, *, epi: int = EPI_NONE, alpha: float = 1.0, bias=None, out_type: int = OUT_F32,
+                   splits: int = 1, c0: bool = False, c_group: int = 0, c_drop: int = 0, force_bn: int = 0, force_stages: int = 0,
+                   rotate: int = 1, c_init=None):
+        """One GEMM of the step as an operator (nsb_op_gemm_ex, include/nsb200.h) -> (y, guard_bad). y: [m_out, n_out] float32, or
+        uint16 bits for 16-bit outputs; EPI_PARTIAL: every k-slice plane [splits, m_out, n_out] float32 (plane 0 from C0 when c0)."""
+        x = np.ascontiguousarray(x, dtype=np.float32)
+        rows = x.shape[0]
+        m_out = rows // c_group * (c_group - c_drop) if c_group else rows
+        keep = []
+        def ptr(a):
+            if a is None:
+                return None
+            a = np.ascontiguousarray(a, dtype=np.float32); keep.append(a)
+            return a.ctypes.data_as(C.c_void_p)
+        op = GemmOp(weight_name.encode(), rows, epi, alpha, out_type, splits, int(c0), c_group, c_drop, force_bn, force_stages, rotate,
+                    ptr(bias), ptr(c_init))
+        n_cap = 4096
+        shape = (splits, m_out, n_cap) if epi == EPI_PARTIAL else (m_out, n_cap)
+        y = np.empty(shape, dtype=np.float32 if out_type == OUT_F32 else np.uint16)
+        bad = C.c_longlong(-1)
+        n = _check(lib().nsb_op_gemm_ex(self.h, C.byref(op), x, y.ctypes.data_as(C.c_void_p), y.nbytes, C.byref(bad)))
+        y = y.reshape(-1)[: int(np.prod(shape[:-1])) * n].reshape(shape[:-1] + (n,)).copy()
+        return y, bad.value
+
+    def op_layernorm(self, x: np.ndarray, g1, b1, *, planes=None, alpha: float = 1.0, fused: bool = False, g2=None, b2=None,
+                     out_type: int = OUT_F32):
+        """The step's LayerNorm launch (nsb_op_layernorm, include/nsb200.h) -> (x after the launch, y float32 or uint16 bits)."""
+        x = np.ascontiguousarray(x, dtype=np.float32)
+        rows = x.shape[0]
+        f = lambda a: None if a is None else np.ascontiguousarray(a, dtype=np.float32)
+        planes, g1, b1, g2, b2 = f(planes), f(g1), f(b1), f(g2), f(b2)
+        vp = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
+        x_out = np.empty_like(x)
+        y = np.zeros((rows, 1024), dtype=np.float32 if out_type == OUT_F32 else np.uint16)
+        n_planes = 0 if planes is None else planes.shape[0]
+        _check(lib().nsb_op_layernorm(self.h, x, rows, vp(planes), n_planes, alpha, g1, b1, vp(g2), vp(b2), int(fused), out_type, x_out,
+                                      y.ctypes.data_as(C.c_void_p)))
+        return x_out, y
 
     def transcribe_full(self, pcm: np.ndarray, want_enc: bool = True, want_frames: bool = False):
         """Non-streaming batch path (nsb_transcribe_full, include/nsb200.h): one whole utterance ->

@@ -166,6 +166,14 @@ int nsb_op_logmel(nsb_engine* e, const int16_t* pcm, int ns, int n, float* out, 
 int nsb_op_gemm(nsb_engine* e, const char* name, const float* x, int rows, float* y, size_t cap) {
     if (!e || !name || !x || !y) return fail(NSB_ERR_ARG, "bad argument"); NSB_TRY return (int)e->impl->op_gemm(name, x, rows, y, cap); NSB_CATCH }
 
+int nsb_op_gemm_ex(nsb_engine* e, const nsb_gemm_op* op, const float* x, void* y, size_t y_bytes, long long* guard_bad) {
+    if (!e || !op || !op->weight || !x || !y) return fail(NSB_ERR_ARG, "bad argument");
+    NSB_TRY return (int)e->impl->op_gemm_ex(*op, x, y, y_bytes, guard_bad); NSB_CATCH }
+int nsb_op_layernorm(nsb_engine* e, const float* x, int rows, const float* planes, int n_planes, float alpha, const float* g1, const float* b1,
+                     const float* g2, const float* b2, int fused, int out_type, float* x_out, void* y) {
+    if (!e || !x || !x_out || !y) return fail(NSB_ERR_ARG, "bad argument");
+    NSB_TRY e->impl->op_layernorm(x, rows, planes, n_planes, alpha, g1, b1, g2, b2, fused != 0, out_type, x_out, y); return NSB_OK; NSB_CATCH }
+
 int nsb_transcribe_full(nsb_engine* e, const int16_t* pcm, int n, int32_t* tokens, int32_t* token_frames, int cap, int* n_frames, float* enc_out, size_t enc_cap) {
     if (!e || !pcm) return fail(NSB_ERR_ARG, "bad argument"); NSB_TRY return (int)e->impl->transcribe_full(pcm, n, tokens, token_frames, cap, n_frames, enc_out, enc_cap); NSB_CATCH }
 

@@ -358,8 +358,9 @@ void Engine::load_weights(const GgufFile& g) {
     // matrices every GGUF keeps in F32: fp32 SIMT in strict mode; on the tensor cores (16-bit / Q8_0 modes) as 3xTF32 -- the
     // split copy [hi | lo | hi] goes to `scales` (NSB_STEM_TF32=1: single-pass tf32 on the plain copy, for A/B measurements)
     auto f32_weight = [&](Weight& w, const std::string& n, int n_out, int n_in, std::vector<float> h) {
-        w.name = n; w.n_out = n_out; w.n_in = n_in; upload(w.data, h);
+        w.name = n; w.n_out = n_out; w.n_in = n_in; w.f32 = true; upload(w.data, h);
         if (!strict() && tf32x3_enabled()) upload(w.scales, tf32x3_weight(h, n_out, n_in));
+        named_[n] = &w;
     };
     // ---- front-end tables (src/preprocessor.cpp:80-110, :296-299) ----
     {
@@ -558,11 +559,16 @@ void Engine::build_pos_tables(const GgufFile& g) {
 
 void Engine::gemm(const void* A, long long lda, const Weight& W, int M, const float* bias, void* C, long long ldc, int epi, float alpha,
                   int out_type) {
-    GemmArgs a; a.A = A; a.lda = lda; a.W = W.data.p; a.w_scales = W.scales.p; a.q4 = W.q4; a.M = M; a.N = W.n_out; a.K = W.n_in; a.bias = bias; a.C = C; a.ldc = ldc;
-    a.epi = epi; a.alpha = alpha; a.out_type = out_type; a.pair = 1; a.q4 = W.q4;
+    GemmArgs a; a.A = A; a.lda = lda; a.M = M; a.bias = bias; a.C = C; a.ldc = ldc;
+    a.epi = epi; a.alpha = alpha; a.out_type = out_type; a.pair = 1;
+    gemm(a, W);
+}
+
+void Engine::gemm(GemmArgs& a, const Weight& W) {
+    a.W = W.data.p; a.w_scales = W.scales.p; a.q4 = W.q4; a.N = W.n_out; a.K = W.n_in;
     ProfScope ps(this, PC_GEMM);
     if (cur_shadow_ && W.shadow_slot >= 0) { a.W = cur_shadow_ + shadow_off_[W.shadow_slot]; a.w_scales = nullptr; a.q4 = 0; }   // dequantised a layer ahead
-    else q8_predequant(W, M, a);
+    else q8_predequant(W, a.M, a);
     if (compute == NSB_COMPUTE_Q8_0_STRICT) { launch_gemm_q8_strict(a, q8s_scratch_.p, q8s_scratch_.bytes, st_); count_launch(); }
     else if (compute == NSB_COMPUTE_F32) launch_gemm_simt(a, st_);
     else launch_gemm_tc(a, act_type(), st_);
@@ -1499,21 +1505,147 @@ long long Engine::transcribe_full(const int16_t* pcm, int n_samples, int32_t* to
     return n_tok;
 }
 
-long long Engine::op_gemm(const std::string& name, const float* xh, int rows, float* y, size_t cap) {
+// The op_* GEMMs below take the weight's A operand the way the step's producers leave it: rounded to the activation type for the
+// per-layer matrices, plain f32 for the F32 matrices (3xTF32 splits it, strict modes run SIMT fp32).
+const Weight& Engine::op_weight(const std::string& name) const {
     auto it = named_.find(name);
     if (it == named_.end()) throw std::invalid_argument("op_gemm: unknown weight '" + name + "'");
+    return *it->second;
+}
+const void* Engine::op_operand(const Weight& W, const float* xh, int rows, DevBuf& dx, DevBuf& da) {
+    dx.alloc((size_t)rows * W.n_in * 4, false);
+    h2d_sync(dx.p, xh, dx.bytes);
+    if (W.f32 || act_type() == OUT_F32) return dx.p;
+    da.alloc((size_t)rows * W.n_in * 2, false);
+    convert_to(dx.as<float>(), da.p, (size_t)rows * W.n_in, act_type(), st_);
+    return da.p;
+}
+// F32 matrices: gemm_f32w splits A into a3_, which the step sizes for its own batch; a larger operator call borrows a scratch of its
+// own for the duration (a3_ itself stays where the captured step graphs expect it)
+struct Engine::SplitScratch {
+    Engine* e; DevBuf tmp; bool swapped = false;
+    SplitScratch(Engine* e_, const Weight& W, int rows) : e(e_) {
+        const size_t need = (size_t)rows * 2 * W.n_in * 4;
+        if (!W.f32 || !W.scales.p || e->a3_.bytes >= need) return;
+        tmp.alloc(need, false); std::swap(e->a3_, tmp); swapped = true;
+    }
+    ~SplitScratch() { if (swapped) { cudaStreamSynchronize(e->st_); std::swap(e->a3_, tmp); } }
+};
+
+long long Engine::op_gemm(const std::string& name, const float* xh, int rows, float* y, size_t cap) {
+    const Weight& W = op_weight(name);
     NSB_CUDA(cudaSetDevice(device_));
-    const Weight& W = *it->second;
     if (cap < (size_t)rows * W.n_out) return -(long long)((size_t)rows * W.n_out);
     ensure_q8s_scratch(rows);
-    DevBuf dx, da, dy; dx.alloc((size_t)rows * W.n_in * 4, false); dy.alloc((size_t)rows * W.n_out * 4, false);
-    h2d_sync(dx.p, xh, dx.bytes);
-    const void* A = dx.p;
-    if (act_type() != OUT_F32) { da.alloc((size_t)rows * W.n_in * 2, false); convert_to(dx.as<float>(), da.p, (size_t)rows * W.n_in, act_type(), st_); A = da.p; }
-    gemm(A, W.n_in, W, rows, nullptr, dy.p, W.n_out, EPI_NONE, 1.f, OUT_F32);
+    DevBuf dx, da, dy; dy.alloc((size_t)rows * W.n_out * 4, false);
+    const void* A = op_operand(W, xh, rows, dx, da);
+    if (W.f32) {
+        SplitScratch sc(this, W, rows);
+        GemmArgs g; g.A = A; g.lda = W.n_in; g.W = W.data.p; g.M = rows; g.N = W.n_out; g.K = W.n_in; g.C = dy.p; g.ldc = W.n_out; g.epi = EPI_NONE;
+        gemm_f32w(g, W, false);
+    } else gemm(A, W.n_in, W, rows, nullptr, dy.p, W.n_out, EPI_NONE, 1.f, OUT_F32);
     NSB_CUDA(cudaStreamSynchronize(st_));
     NSB_CUDA(cudaMemcpy(y, dy.p, dy.bytes, cudaMemcpyDeviceToHost));
     return W.n_out;
+}
+
+namespace {
+constexpr int GUARD_ROWS = 128;            // guard rows before and after every destination of op_gemm_ex: one whole row tile each way
+constexpr int GUARD_COLS = 32;             // unused columns per row (ldc = N + 32)
+constexpr uint32_t GUARD_WORD = 0x7FDA7FDAu;   // NaN as f32, and each half a NaN as f16 and as bf16
+
+// a destination of op_gemm_ex: `live` rows of `cols` elements at row stride cols + GUARD_COLS, between GUARD_ROWS guard rows
+struct Guarded {
+    DevBuf d; size_t es = 4, ld = 0, live = 0, cols = 0;
+    void init(size_t live_rows, size_t n, size_t elem, const float* live_init) {
+        es = elem; ld = n + GUARD_COLS; live = live_rows; cols = n;
+        std::vector<uint8_t> h(bytes());
+        for (size_t i = 0; i + 4 <= h.size(); i += 4) memcpy(&h[i], &GUARD_WORD, 4);
+        if (live_init)
+            for (size_t r = 0; r < live; ++r) memcpy(&h[((GUARD_ROWS + r) * ld) * es], live_init + r * n, n * 4);
+        d.alloc(h.size(), false); h2d_sync(d.p, h.data(), h.size());
+    }
+    size_t bytes() const { return (2 * GUARD_ROWS + live) * ld * es; }
+    void* at() const { return (char*)d.p + GUARD_ROWS * ld * es; }
+    // copies the live rows (packed, n elements each) to out and returns how many guard elements differ from the pattern
+    long long fetch(void* out) const {
+        std::vector<uint8_t> h(bytes());
+        NSB_CUDA(cudaMemcpy(h.data(), d.p, h.size(), cudaMemcpyDeviceToHost));
+        long long bad = 0;
+        for (size_t r = 0; r < 2 * GUARD_ROWS + live; ++r) {
+            const bool live_row = r >= GUARD_ROWS && r < GUARD_ROWS + live;
+            for (size_t c = live_row ? cols : 0; c < ld; ++c) bad += memcmp(&h[(r * ld + c) * es], &GUARD_WORD, es) != 0;
+            if (live_row) memcpy((char*)out + (r - GUARD_ROWS) * cols * es, &h[r * ld * es], cols * es);
+        }
+        return bad;
+    }
+};
+}  // namespace
+
+long long Engine::op_gemm_ex(const nsb_gemm_op& op, const float* xh, void* y, size_t y_bytes, long long* guard_bad) {
+    const Weight& W = op_weight(op.weight);
+    const int rows = op.rows, N = W.n_out;
+    auto bad = [](const std::string& m) { throw std::invalid_argument("op_gemm_ex: " + m); };
+    if (rows < 1) bad("rows must be >= 1");
+    if (op.epi < EPI_NONE || op.epi > EPI_PARTIAL) bad("unknown epilogue");
+    if (op.out_type < OUT_F32 || op.out_type > OUT_BF16) bad("unknown output type");
+    if (op.out_type != OUT_F32 && (op.epi == EPI_RESID || op.epi == EPI_PARTIAL)) bad("residual and split-K outputs are f32");
+    if (op.splits < 1 || op.splits > MAX_SPLITS || (op.splits > 1 && op.epi != EPI_PARTIAL)) bad("splits must be 1..8, > 1 only with the split-K epilogue");
+    if (op.c0 && op.epi != EPI_PARTIAL) bad("c0 is a split-K destination");
+    if (op.c_group < 0 || (op.c_group > 0 && (op.c_drop < 0 || op.c_drop >= op.c_group || rows % op.c_group != 0))) bad("bad output row map");
+    if (op.epi == EPI_RESID && !op.c_init) bad("the residual epilogue needs c_init");
+    if (strict() && (op.out_type != OUT_F32 || op.epi == EPI_PARTIAL || op.c_group || op.force_bn))
+        bad("strict modes run the SIMT / Q8_0 block kernels: f32 output, no split-K, row map or tile config");
+    NSB_CUDA(cudaSetDevice(device_));
+    const int m_out = op.c_group > 0 ? rows / op.c_group * (op.c_group - op.c_drop) : rows;
+    const bool partial = op.epi == EPI_PARTIAL;
+    const size_t es = out_elem_size(op.out_type), need = partial ? (size_t)op.splits * m_out * N * 4 : (size_t)m_out * N * es;
+    if (y_bytes < need) return -(long long)need;
+    ensure_q8s_scratch(rows);
+    DevBuf dx, da, dbias;
+    const void* A = op_operand(W, xh, rows, dx, da);
+    if (op.bias) { dbias.alloc((size_t)N * 4, false); h2d_sync(dbias.p, op.bias, dbias.bytes); }
+    // destinations: C (or, split-K, the workspace of the slices that do not go to C0) and C0
+    const int ws_planes = partial ? op.splits - (op.c0 ? 1 : 0) : 1;
+    Guarded c, c0;
+    c.init((size_t)ws_planes * m_out, N, partial ? 4 : es, op.epi == EPI_RESID ? op.c_init : nullptr);
+    if (op.c0) c0.init(m_out, N, 4, nullptr);
+
+    GemmArgs g; g.A = A; g.lda = W.n_in; g.W = W.data.p; g.M = rows; g.N = N; g.K = W.n_in; g.bias = op.bias ? dbias.as<float>() : nullptr;
+    g.C = c.at(); g.ldc = (long long)c.ld; g.epi = op.epi; g.alpha = op.alpha; g.out_type = op.out_type; g.splits = op.splits;
+    g.c_group = op.c_group; g.c_drop = op.c_drop; g.C0 = op.c0 ? c0.at() : nullptr; g.force_bn = op.force_bn; g.force_stages = op.force_stages;
+    g.rotate = op.rotate; g.pair = 1;
+    if (W.f32) { SplitScratch sc(this, W, rows); gemm_f32w(g, W, false); NSB_CUDA(cudaStreamSynchronize(st_)); }
+    else gemm(g, W);
+    NSB_CUDA(cudaStreamSynchronize(st_));
+    long long nbad = 0;
+    if (op.c0) nbad += c0.fetch(y);
+    nbad += c.fetch((char*)y + (op.c0 ? (size_t)m_out * N * 4 : 0));
+    if (guard_bad) *guard_bad = nbad;
+    return N;
+}
+
+void Engine::op_layernorm(const float* xh, int rows, const float* planes, int n_planes, float alpha, const float* g1, const float* b1,
+                          const float* g2, const float* b2, bool fused, int out_type, float* x_out, void* y) {
+    // load_x_reduced folds at most MAX_SPLITS planes: every split-K producer stays within that
+    if (rows < 1 || n_planes < 0 || n_planes > MAX_SPLITS || (n_planes && !planes) || !g1 || !b1 || (!g2) != (!b2) || (g2 && !fused))
+        throw std::invalid_argument("op_layernorm: bad arguments (rows >= 1, 0..8 planes, g1 / b1, g2 / b2 together and only fused)");
+    if (out_type < OUT_F32 || out_type > OUT_BF16) throw std::invalid_argument("op_layernorm: unknown output type");
+    NSB_CUDA(cudaSetDevice(device_));
+    const size_t n = (size_t)rows * D_MODEL;
+    auto up = [](DevBuf& d, const float* h, size_t count) { d.alloc(count * 4, false); h2d_sync(d.p, h, count * 4); };
+    DevBuf dx, dp, dg1, db1, dg2, db2, dy;
+    up(dx, xh, n); up(dg1, g1, D_MODEL); up(db1, b1, D_MODEL);
+    if (n_planes) up(dp, planes, (size_t)n_planes * n);
+    if (g2) { up(dg2, g2, D_MODEL); up(db2, b2, D_MODEL); }
+    dy.alloc(n * out_elem_size(out_type), false);
+    PartialSum ps; ps.part = n_planes ? dp.as<float>() : nullptr; ps.n = n_planes; ps.alpha = alpha;
+    if (!fused) launch_layernorm(dx.as<float>(), rows, dg1.as<float>(), db1.as<float>(), dy.p, out_type, ps, st_);
+    else launch_layernorm2(dx.as<float>(), rows, dg1.as<float>(), db1.as<float>(), dg2.as<float>(), db2.as<float>(), g2 ? dy.p : nullptr,
+                           out_type, ps, st_);
+    NSB_CUDA(cudaStreamSynchronize(st_));
+    NSB_CUDA(cudaMemcpy(x_out, dx.p, n * 4, cudaMemcpyDeviceToHost));
+    if (y && (!fused || g2)) NSB_CUDA(cudaMemcpy(y, dy.p, dy.bytes, cudaMemcpyDeviceToHost));
 }
 
 }  // namespace nsb

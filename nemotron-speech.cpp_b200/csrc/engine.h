@@ -42,6 +42,7 @@ struct Weight {
     std::string name; int n_out = 0, n_in = 0;
     int q4 = 0;             // Q8_0 mode, Q4_0 file: `data` is the nibble plane [n_out][n_in / 2] (fused-dequant GEMM variant)
     int shadow_slot = -1;   // Q8_0 mode: which of the layer's 8 matrices this is (offset into the fp16 shadow of the layer, see Engine::shadow_)
+    bool f32 = false;       // kept in F32 by every GGUF (stem 1x1 convs and projection, joint.enc): Engine::gemm_f32w
     DevBuf data;            // f32 / f16 / bf16 [n_out][n_in]; Q8_0 mode: int8 quants [n_out][n_in]
     DevBuf scales;          // Q8_0 mode only: fp16 block scales [n_out][n_in / 32]
 };
@@ -94,6 +95,9 @@ public:
     long long debug_get_cache(int stream, int which, int layer, float* out, size_t cap);
     long long op_logmel(const int16_t* pcm, int n_streams, int n_samples, float* out, size_t cap);
     long long op_gemm(const std::string& name, const float* x, int rows, float* y, size_t cap);
+    long long op_gemm_ex(const nsb_gemm_op& op, const float* x, void* y, size_t y_bytes, long long* guard_bad);
+    void op_layernorm(const float* x, int rows, const float* planes, int n_planes, float alpha, const float* g1, const float* b1,
+                      const float* g2, const float* b2, bool fused, int out_type, float* x_out, void* y);
     // Non-streaming batch path (nemo_encode, reference src/nemo-ggml.cpp:1467-1535) for one utterance: whole-utterance log-mel ->
     // un-chunked subsampling -> non-cached layers with full-context rel-pos attention -> greedy decode from a fresh decoder state.
     // Borrows one free stream slot (decoder / conv state); the activations live in a workspace of their own, grown to the longest
@@ -124,9 +128,14 @@ private:
     std::vector<DevBuf> full_pos_; int full_pos_cap_ = 0;
     void gemm(const void* A, long long lda, const Weight& W, int M, const float* bias, void* C, long long ldc, int epi, float alpha,
               int out_type);
+    void gemm(GemmArgs& a, const Weight& W);   // the launch behind gemm() for explicit GemmArgs (A, M, C, epilogue set by the caller)
     // x += alpha * A W^T. Small batches: split-K into the workspace, reduction folded into the next LayerNorm (pending_).
     void gemm_residual(const void* A, long long lda, const Weight& W, int M, float* x, float alpha);
     bool split_consumers(int rows) const;
+    // operator entry points (op_gemm, op_gemm_ex): weight by name, A operand as the step's producers leave it, split scratch of F32 matrices
+    const Weight& op_weight(const std::string& name) const;
+    const void* op_operand(const Weight& W, const float* xh, int rows, DevBuf& dx, DevBuf& da);
+    struct SplitScratch;
     void q8_predequant(const Weight& W, int M, GemmArgs& a);
     void gemm_f32w(GemmArgs& g, const Weight& W, bool a_presplit);   // matrices kept in F32 by every GGUF: SIMT fp32 / 3xTF32
     void gemm_planes(const void* A, long long lda, const Weight& W, int M, void* C, int planes);

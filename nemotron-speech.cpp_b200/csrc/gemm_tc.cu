@@ -19,7 +19,10 @@
 #include <cuda.h>
 
 #include <algorithm>
+#include <initializer_list>
 #include <mutex>
+#include <stdexcept>
+#include <string>
 
 #include "kernels.cuh"
 
@@ -1166,6 +1169,11 @@ CUtensorMap make_map_u8(const void* ptr, int rows, int K, int box_rows, int box_
     return m;
 }
 
+// the single-CTA and 128-row pair tiles launch N / BN column tiles: with N % BN != 0 the last columns would never be written
+void require_full_grid(int N, int BN) {
+    if (N % BN != 0) throw std::invalid_argument("gemm_tc: N = " + std::to_string(N) + " is not a multiple of the tile width " + std::to_string(BN));
+}
+
 template <int BN, int STAGES, int Q4>
 void launch_cfg_q8x(const GemmArgs& a, cudaStream_t st) {
     static std::atomic<size_t> attr_set[MAX_DEVICES];
@@ -1174,6 +1182,7 @@ void launch_cfg_q8x(const GemmArgs& a, cudaStream_t st) {
     if (a.K / 64 / a.splits > 64) throw CudaError("gemm_q8: k range per CTA too long for the scale buffer");
     const CUtensorMap tmA = make_map(a.A, a.M, a.K, a.lda, BM, 0);
     const CUtensorMap tmQ = Q4 ? make_map_u8(a.W, a.N, a.K / 2, BN, 32) : make_map_u8(a.W, a.N, a.K, BN);
+    require_full_grid(a.N, BN);
     const int m_out = a.c_group > 0 ? (a.M / a.c_group) * (a.c_group - a.c_drop) : a.M;
     TcParams p{a.M, a.N, a.K, a.bias, a.C, a.ldc, a.epi, a.alpha, a.out_type, 0, a.rotate, a.c_group, a.c_drop, a.C0, m_out};
     dim3 grid(a.N / BN, (a.M + BM - 1) / BM, a.splits);
@@ -1214,6 +1223,7 @@ bool multicast_enabled() {
 template <int BN, int STAGES, int EB, int CL>
 void launch_cfg_c(const GemmArgs& a, int fmt, cudaStream_t st) {
     static std::atomic<size_t> attr_set[MAX_DEVICES];
+    require_full_grid(a.N, BN);
     const size_t smem = sizeof(Smem<BN, STAGES>) + 1024;
     ensure_dyn_smem(gemm_tc_kernel<BN, STAGES, EB, CL>, smem, attr_set);
     const CUtensorMap tmA = make_map(a.A, a.M, a.a_fold ? 2 * a.a_fold : a.K, a.lda, BM / CL, fmt);
@@ -1226,6 +1236,7 @@ void launch_cfg_c(const GemmArgs& a, int fmt, cudaStream_t st) {
 template <int BN, int STAGES>
 void launch_cfg_pair(const GemmArgs& a, int fmt, cudaStream_t st) {
     static std::atomic<size_t> attr_set[MAX_DEVICES];
+    require_full_grid(a.N, BN);
     const size_t smem = sizeof(SmemPair<BN, STAGES>) + 1024;
     ensure_dyn_smem(gemm_tc_pair_kernel<BN, STAGES>, smem, attr_set);
     const CUtensorMap tmA = make_map(a.A, a.M, a.K, a.lda, 64, fmt);
@@ -1313,6 +1324,34 @@ void launch_pair256(const GemmArgs& a, int fmt, int bn, cudaStream_t st) {
         case 112: launch_cfg_pair256<112, 4>(a, fmt, st); break;
         default: throw CudaError("gemm_tc: pair256 tile not instantiated");
     }
+}
+
+// A forced tile config (nsb_bench_gemm, nsb_op_gemm_ex) must name a tile the dispatch below instantiates for this operand type, and the
+// tile's grid must cover all N columns; anything else is the caller's error, not a launch that computes part of C.
+void check_forced_config(const GemmArgs& a, int fmt) {
+    const int bn = a.force_bn, st = a.force_stages;
+    auto fail = [&](const char* why) {
+        throw std::invalid_argument("gemm_tc: forced tile " + std::to_string(bn) + "/" + std::to_string(st) + ": " + why);
+    };
+    auto one_of = [](int v, std::initializer_list<int> l) { return std::find(l.begin(), l.end(), v) != l.end(); };
+    if (a.w_scales) {                                             // fused Q8_0 / Q4_0 planes: only the 256-row pair tiles (grid rounds up along N)
+        if (st != 95 || !one_of(bn, {112, 160, 208})) fail("not instantiated for Q8_0 / Q4_0 planes");
+        return;
+    }
+    if (st == 95) fail("the fused Q8_0 tiles need Q8_0 / Q4_0 planes");
+    if (st == 96 || st == 97) {                                   // 256-row pair tiles: grid rounds up along N, the epilogue clips the last tile
+        if (fmt == 2) fail("pair tiles are 16-bit only");
+        if (!one_of(bn, st == 97 ? std::initializer_list<int>{112, 160, 208, 256} : std::initializer_list<int>{112, 128, 160, 208, 256})) fail("not instantiated");
+        return;
+    }
+    const int key = bn * 100 + st;
+    if (!one_of(key, {3204, 3205, 3208, 6404, 6498, 6406, 12803, 12804, 25602, 25603})) fail("not instantiated");
+    if (fmt == 2 && !one_of(key, {3205, 6404, 12803, 12804, 25602})) fail("not instantiated for tf32");
+    if (a.N % bn != 0) fail("the grid does not cover N");
+}
+void check_splits(const GemmArgs& a, int BK) {
+    if (a.splits > 1 && (a.epi != EPI_PARTIAL || (a.K / BK) % a.splits != 0))
+        throw std::invalid_argument("gemm_tc: bad split-K request (" + std::to_string(a.splits) + " slices of " + std::to_string(a.K / BK) + " k-blocks)");
 }
 
 template <int BN, int STAGES, int EB>
@@ -1409,8 +1448,8 @@ void launch_gemm_tc(const GemmArgs& a, int in_type, cudaStream_t st) {
     const int tiles_m = (a.M + BM - 1) / BM;
     if (a.w_scales) {                                             // Q8_0 planes: fused-dequant kernel (A is fp16)
         if (fmt != 0) throw CudaError("gemm_q8: activations must be fp16");
-        if (a.splits > 1 && (a.epi != EPI_PARTIAL || (a.K / BK) % a.splits != 0)) throw CudaError("gemm_tc: bad split-K request");
-        if (a.force_bn && a.force_stages == 95) { launch_q8_pair256(a, a.force_bn, st); return; }      // tuning hook
+        check_splits(a, BK);
+        if (a.force_bn) { check_forced_config(a, fmt); launch_q8_pair256(a, a.force_bn, st); return; }      // tuning hook
         if (tiles_m >= pair256_min_tiles() && q8_pair256_enabled()) {   // large batches: fused dequantisation on the 256-row CTA-pair tiles
             static const int split_bn = [] { const char* e = getenv("NSB_SPLIT_BN"); return e ? atoi(e) : 112; }();
             const int bn = a.splits > 1 ? (split_bn == 256 ? 208 : split_bn) : pick_q8_pair256_bn(a.M, a.N);
@@ -1423,16 +1462,17 @@ void launch_gemm_tc(const GemmArgs& a, int in_type, cudaStream_t st) {
         return;
     }
     if (a.force_bn) {                                             // tuning hook
-        if (a.splits > 1 && (a.epi != EPI_PARTIAL || (a.K / BK) % a.splits != 0)) throw CudaError("gemm_tc: bad split-K request");
-        if (a.force_stages == 97) { if (fmt == 2) throw CudaError("gemm_tc: pair tiles are 16-bit only"); launch_pair256(a, fmt, a.force_bn, st); return; }
-        if (a.force_stages == 96) { if (fmt == 2) throw CudaError("gemm_tc: pair tiles are 16-bit only"); launch_pair256_persist(a, fmt, a.force_bn, st); return; }
+        check_splits(a, BK);
+        check_forced_config(a, fmt);
+        if (a.force_stages == 97) { launch_pair256(a, fmt, a.force_bn, st); return; }
+        if (a.force_stages == 96) { launch_pair256_persist(a, fmt, a.force_bn, st); return; }
         const int key = a.force_bn * 100 + a.force_stages;
         switch (key) {
             case 3204: launch_cfg<32, 4>(a, fmt, st); break;
             case 3205: launch_cfg<32, 5>(a, fmt, st); break;
             case 3208: launch_cfg<32, 8>(a, fmt, st); break;
             case 6404: launch_cfg<64, 4>(a, fmt, st); break;
-            case 6498: if (fmt == 2) throw CudaError("gemm_tc: pair tiles are 16-bit only"); launch_cfg_pair<64, 8>(a, fmt, st); break;
+            case 6498: launch_cfg_pair<64, 8>(a, fmt, st); break;
             case 6406: launch_cfg<64, 6>(a, fmt, st); break;
             case 12803: launch_cfg<128, 3>(a, fmt, st); break;
             case 12804: launch_cfg<128, 4>(a, fmt, st); break;
@@ -1443,7 +1483,7 @@ void launch_gemm_tc(const GemmArgs& a, int in_type, cudaStream_t st) {
         return;
     }
     if (a.splits > 1) {
-        if (a.epi != EPI_PARTIAL || (a.K / BK) % a.splits != 0) throw CudaError("gemm_tc: bad split-K request");
+        check_splits(a, BK);
         if (fmt != 2 && tiles_m >= 8 && pair256_enabled()) {            // large-batch split-K (FFN down): wide pair tiles
             static const int bn = [] { const char* e = getenv("NSB_SPLIT_BN"); return e ? atoi(e) : 112; }();
             if (pair256_persist_enabled()) launch_pair256_persist(a, fmt, bn, st); else launch_pair256(a, fmt, bn, st);
