@@ -103,6 +103,23 @@ int nsb_stream_open(nsb_engine* e);                /* returns stream id >= 0, or
 int nsb_stream_close(nsb_engine* e, int stream);
 int nsb_stream_reset(nsb_engine* e, int stream);   /* re-zeroes caches too (the reference's reset does not) */
 
+/* ---- stream snapshots: suspend, resume and move live streams (no counterpart in the reference) --------------------------
+ * A snapshot holds everything that decides the stream's future output: its K/V ring, conv state, mel overlap and decoder state,
+ * the PCM buffered for chunks not yet launched, its chunk counters and the tokens not yet popped. Engine statistics are not part
+ * of it. Callers treat it as opaque bytes (layout: DESIGN.md §11). Both calls collect the steps in flight first, like open / close.
+ * nsb_stream_export: the stream stays open and continues exactly as if nothing happened (tokens of the steps that were in flight
+ *   are in the snapshot and stay poppable on the stream). out == NULL: returns the size an export would write now. Returns the
+ *   bytes written; a closed stream, an invalid id, or cap smaller than the size is NSB_ERR_ARG (the buffer is left untouched).
+ *   Suspend = export, then close; move = export on A, import on B, close on A.
+ * nsb_stream_import: takes the lowest free slot like nsb_stream_open and returns the new stream id. The engine must run the same
+ *   model (a fingerprint of the GGUF: metadata, tensor table, first and last 4 KiB of every tensor -- the path does not matter),
+ *   n_layers, att_right_context, kv_dtype and resolved compute; device, max_streams, use_cuda_graph and decode_overlap may differ.
+ *   NSB_ERR_FORMAT: not a valid snapshot (magic, version, size, checksum, a field out of range); NSB_ERR_ARG: a valid snapshot that
+ *   does not fit this engine; NSB_ERR_STATE: no free slot. nsb_last_error() names the field. A failed import changes nothing:
+ *   no slot is consumed and no other stream is touched. */
+long long nsb_stream_export(nsb_engine* e, int stream, void* out, size_t cap);
+int nsb_stream_import(nsb_engine* e, const void* snapshot, size_t bytes);
+
 /* ---- the hot call: replaces nemo_stream_process_incremental (src/nemo-stream.cpp:1074-1134)
  *      split into push (buffer PCM, any length) / step (one batched chunk for every stream that
  *      has a full chunk buffered) / pop (token ids decoded so far). ------------------------- */

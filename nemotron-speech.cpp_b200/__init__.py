@@ -59,7 +59,7 @@ EXPORTS = ["nsb_gguf_probe", "nsb_gguf_read_tensor", "nsb_default_config", "nsb_
            "nsb_stream_open", "nsb_stream_close", "nsb_stream_reset", "nsb_stream_push_pcm", "nsb_push_pcm_batch", "nsb_pop_tokens_batch", "nsb_stream_ready", "nsb_engine_step", "nsb_engine_step_begin", "nsb_engine_step_end",
            "nsb_engine_drain", "nsb_stream_pop_tokens", "nsb_stream_chunks", "nsb_detokenize", "nsb_engine_get_stats",
            "nsb_bench_prepare", "nsb_bench_step", "nsb_bench_steps", "nsb_bench_profile", "nsb_profiler_range", "nsb_bench_gemm", "nsb_trace_enable", "nsb_trace_fetch", "nsb_debug_enable", "nsb_debug_get", "nsb_debug_get_cache", "nsb_op_logmel",
-           "nsb_op_gemm", "nsb_op_gemm_ex", "nsb_op_layernorm", "nsb_transcribe_full"]
+           "nsb_op_gemm", "nsb_op_gemm_ex", "nsb_op_layernorm", "nsb_transcribe_full", "nsb_stream_export", "nsb_stream_import"]
 
 
 def build(force: bool = False) -> str:
@@ -97,6 +97,9 @@ def lib():
         L.nsb_engine_vocab.restype = vp
         for n in ("nsb_stream_close", "nsb_stream_reset", "nsb_stream_ready", "nsb_stream_chunks"):
             getattr(L, n).argtypes = [vp, ci]
+        L.nsb_stream_export.argtypes = [vp, ci, vp, C.c_size_t]
+        L.nsb_stream_export.restype = C.c_longlong
+        L.nsb_stream_import.argtypes = [vp, C.c_char_p, C.c_size_t]
         L.nsb_stream_push_pcm.argtypes = [vp, ci, _i16p, ci]
         L.nsb_stream_pop_tokens.argtypes = [vp, ci, _i32p, ci]
         L.nsb_push_pcm_batch.argtypes = [vp, ci, _i32p, _i16p, ci, ci]
@@ -184,6 +187,18 @@ class Engine:
 
     def reset_stream(self, s: int):
         _check(lib().nsb_stream_reset(self.h, s))
+
+    def export_stream(self, s: int) -> bytes:
+        """Snapshot of an open stream (nsb_stream_export, include/nsb200.h); the stream stays open and continues unchanged."""
+        n = _check(int(lib().nsb_stream_export(self.h, s, None, 0)))
+        buf = C.create_string_buffer(n)
+        _check(int(lib().nsb_stream_export(self.h, s, buf, n)))
+        return buf.raw
+
+    def import_stream(self, blob: bytes) -> int:
+        """A snapshot from export_stream as a new stream of this engine (nsb_stream_import); returns its id."""
+        blob = bytes(blob)
+        return _check(lib().nsb_stream_import(self.h, blob, len(blob)))
 
     def push(self, s: int, pcm: np.ndarray):
         pcm = np.ascontiguousarray(pcm, dtype=np.int16)

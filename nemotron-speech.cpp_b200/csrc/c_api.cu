@@ -18,6 +18,7 @@ static int fail(int code, const std::string& msg) { g_err = msg; return code; }
 #define NSB_CATCH                                                                         \
     } catch (const nsb::CudaError& e) { return fail(NSB_ERR_CUDA, e.what());              \
     } catch (const std::invalid_argument& e) { return fail(NSB_ERR_ARG, e.what());        \
+    } catch (const nsb::FormatError& e) { return fail(NSB_ERR_FORMAT, e.what());          \
     } catch (const std::bad_alloc&) { return fail(NSB_ERR_NOMEM, "out of host memory");   \
     } catch (const std::exception& e) { return fail(NSB_ERR_STATE, e.what()); }
 
@@ -103,6 +104,10 @@ int nsb_engine_set_cuda_graph(nsb_engine* e, int on) { if (!e) return fail(NSB_E
 int nsb_stream_open(nsb_engine* e) { if (!e) return fail(NSB_ERR_ARG, "null engine"); NSB_TRY return e->impl->open_stream(); NSB_CATCH }
 int nsb_stream_close(nsb_engine* e, int s) { if (!e) return fail(NSB_ERR_ARG, "null engine"); NSB_TRY e->impl->close_stream(s); return NSB_OK; NSB_CATCH }
 int nsb_stream_reset(nsb_engine* e, int s) { if (!e) return fail(NSB_ERR_ARG, "null engine"); NSB_TRY e->impl->reset_stream(s); return NSB_OK; NSB_CATCH }
+long long nsb_stream_export(nsb_engine* e, int s, void* out, size_t cap) {
+    if (!e) return fail(NSB_ERR_ARG, "null engine"); NSB_TRY return e->impl->export_stream(s, out, cap); NSB_CATCH }
+int nsb_stream_import(nsb_engine* e, const void* snapshot, size_t bytes) {
+    if (!e || !snapshot) return fail(NSB_ERR_ARG, "bad argument"); NSB_TRY return e->impl->import_stream(snapshot, bytes); NSB_CATCH }
 int nsb_stream_push_pcm(nsb_engine* e, int s, const int16_t* pcm, int n) {
     if (!e) return fail(NSB_ERR_ARG, "null engine"); NSB_TRY e->impl->push_pcm(s, pcm, n); return NSB_OK; NSB_CATCH }
 int nsb_push_pcm_batch(nsb_engine* e, int n_streams, const int32_t* streams, const int16_t* pcm, int row_stride, int n_samples) {

@@ -204,6 +204,7 @@ Engine::Engine(const std::string& path, const nsb_engine_config& cfg) : cfg_(cfg
         // Q8_0 and Q4_0 files stay quantised in HBM (fused-dequant GEMM; NSB_COMPUTE_F16 on such a file expands it to fp16 at load)
         compute = t == GGML_F32 ? NSB_COMPUTE_F32 : t == GGML_F16 ? NSB_COMPUTE_F16 : NSB_COMPUTE_Q8_0;
     }
+    fingerprint = g.fingerprint();
     load_weights(g);
     alloc_state();
     build_pos_tables(g);

@@ -30,6 +30,11 @@ struct DevBuf {
     template <class T> T* as() const { return (T*)p; }
 };
 
+constexpr int SNAP_BULK = 6;   // bulk device sections of a stream snapshot (stream_state.cu)
+
+// a buffer that is not a valid stream snapshot (nsb_stream_import: NSB_ERR_FORMAT)
+struct FormatError : std::runtime_error { using std::runtime_error::runtime_error; };
+
 struct HostPinned {
     void* p = nullptr; size_t bytes = 0;
     ~HostPinned() { if (p) cudaFreeHost(p); }
@@ -71,6 +76,10 @@ public:
     int step_end();                   // returns #streams advanced (0 = no step in flight)
     int pop_tokens(int s, int32_t* out, int cap);
     int chunks(int s) const;
+    // stream snapshots (stream_state.cu; format in DESIGN.md §11): export leaves the stream open and unchanged, returns the bytes
+    // written (out == nullptr: the size only); import takes the lowest free slot and returns it
+    long long export_stream(int s, void* out, size_t cap);
+    int import_stream(const void* blob, size_t bytes);
     std::string detok(const int32_t* t, int n) const;
 
     void bench_prepare(int n_streams, const int16_t* pcm, int samples_per_stream, int warm_chunks);
@@ -107,6 +116,7 @@ public:
 
     // facts
     int n_layers = 0, T = 1, R = 0, compute = NSB_COMPUTE_F32, kv_dtype = NSB_KV_F32, max_streams = 0;
+    uint64_t fingerprint = 0;         // model identity a snapshot carries (GgufFile::fingerprint)
     std::vector<char> vocab;
     nsb_stats stats{};
     int chunk_samples() const { return (PRE_CACHE + 8 * T) * HOP; }
@@ -204,6 +214,10 @@ private:
     DevBuf ring_pos_, valid_len_;  // [S] int
     DevBuf dec_h_, dec_c_, dec_par_, dec_proj_, prev_token_, cand_valid_;
     std::vector<HostStream> hs_;
+    // snapshots: the slot's bulk arrays as (device pointer, bytes) in snapshot order; returns their total
+    size_t snapshot_sections(int s, void** ptr, size_t* bytes) const;
+    uint64_t device_checksum(void* const* ptr, const size_t* bytes, size_t first_word);   // syncs st_
+    DevBuf snap_sum_;
 
     // ---- step workspace (batch-compact) ----
     int rl_ = 0;                   // PCM row length per stream-step

@@ -1,5 +1,6 @@
 #include "gguf_loader.h"
 
+#include <algorithm>
 #include <cstdio>
 #include <cmath>
 #include <cstring>
@@ -180,6 +181,20 @@ std::vector<float> GgufFile::read_dequant(const std::string& name) const {
         }
     } else throw std::runtime_error("unsupported tensor type for " + name);
     return out;
+}
+
+uint64_t GgufFile::fingerprint() const {
+    uint64_t h = 0xcbf29ce484222325ull;
+    auto eat = [&](const uint8_t* p, size_t n) { for (size_t i = 0; i < n; ++i) { h ^= p[i]; h *= 0x100000001b3ull; } };
+    eat(map, (size_t)std::min<uint64_t>(data_start, map_size));   // magic, metadata, tensor table
+    for (const auto& kv : tensors) {                               // name order
+        const GgufTensor& t = kv.second;
+        const uint8_t* p = data(t);
+        const size_t edge = std::min<size_t>(t.nbytes, 4096);
+        eat(p, edge);
+        eat(p + t.nbytes - edge, edge);
+    }
+    return h;
 }
 
 }  // namespace nsb

@@ -46,6 +46,9 @@ struct GgufFile {
     // (fp16 d + 16 nibble bytes: element i = low nibble of byte i, element i + 16 = high nibble) as d * (q - 8)
     // (scripts/convert_to_gguf.py:93-179; what ggml's dequantize_row_q8_0 / _q4_0 return).
     std::vector<float> read_dequant(const std::string& name) const;
+    // 64-bit FNV-1a over the header (metadata and tensor table) and the first and last 4 KiB of every tensor's bytes: tells models
+    // apart without a pass over the weights, and does not depend on the file's path
+    uint64_t fingerprint() const;
 };
 
 // fp16 bits -> float (host)
