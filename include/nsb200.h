@@ -228,6 +228,32 @@ typedef struct nsb_gemm_op {
     const float* c_init;       /* NSB_EPI_RESID: initial C [m_out][n_out]                                                 */
 } nsb_gemm_op;
 int nsb_op_gemm_ex(nsb_engine* e, const nsb_gemm_op* op, const float* x, void* y, size_t y_bytes, long long* guard_bad);
+/* nsb_op_decode: the step's RNN-T greedy-decode launch (LSTM prediction net, joint.pred, joint, argmax, up to 10 symbols per frame)
+ *   on the engine's decoder weights, for B streams of T frames each. enc_proj [B][T][640] f32 is what joint.enc produced (bias
+ *   included). The decoder state of S >= B slots comes in and goes out in the engine's layout: h, c [S][2 parities][2 layers x 640]
+ *   (committed state at parity par[s], candidate at the other), dec_proj [S][640] (joint.pred projection of the candidate), par,
+ *   prev_token (0..1024), cand_valid (0 / 1) [S]; batch row b decodes slot slot_of_b[b] (distinct). Device state, sync buffer and
+ *   outputs are private to the call: no stream slot is touched. grid = 0: one CTA per SM (cooperative launch, as in a step);
+ *   grid = k (even, 2 <= k < SM count): the decode-overlap launch with k CTAs in pairs. pipe_min_n: streams per phase from which
+ *   the pipelined tiles run on a wide grid (0 = the engine's default). Outputs: tokens / frames [B][10 T] (entries past counts[b]
+ *   keep -1), counts [B], optionally the logits of batch row 0 at each of its joint evaluations, logits [11 T][1025] (*n_logits =
+ *   evaluations), the grid used and the number of guard entries behind the token / frame buffers the launch changed. Runs on the
+ *   engine stream and synchronises. Returns 0, NSB_ERR_ARG for a bad argument (nothing is written then). */
+typedef struct nsb_decode_op {
+    int32_t B, T, S;           /* 1 <= B <= 1024, 1 <= T <= 3276 (10 T emissions fit the kernel's 16-bit counters), B <= S <= 8192 */
+    int32_t grid, pipe_min_n;  /* launch choice (above)                                                                        */
+    const int32_t* slot_of_b;  /* [B]                                                                                          */
+    const float* enc_proj;     /* [B][T][640]                                                                                  */
+    float* h; float* c;        /* in / out [S][2][1280]                                                                        */
+    float* dec_proj;           /* in / out [S][640]                                                                            */
+    int32_t* par; int32_t* prev_token; int32_t* cand_valid;   /* in / out [S]                                                 */
+    int32_t* tokens; int32_t* frames;   /* out [B][10 T]                                                                       */
+    int32_t* counts;           /* out [B]                                                                                      */
+    float* logits;             /* out [11 T][1025] or NULL                                                                     */
+    int32_t n_logits, grid_used;        /* out                                                                                 */
+    long long guard_bad;       /* out                                                                                          */
+} nsb_decode_op;
+int nsb_op_decode(nsb_engine* e, nsb_decode_op* op);
 /* nsb_op_layernorm: the LayerNorm launch of the step on host rows of 1024: x [rows][1024] f32 += alpha * (sum of n_planes split-K
  *   planes [n_planes][rows][1024], 0 <= n_planes <= 8, summed in plane order), then fused = 0: y = LN(x; g1, b1) (x keeps the reduced
  *   rows); fused = 1 (norm_out fused with the next layer's first norm): x = LN(x; g1, b1) and, when g2 is set, y = LN(x; g2, b2).

@@ -49,6 +49,13 @@ class GemmOp(C.Structure):
                 ("force_stages", C.c_int32), ("rotate", C.c_int32), ("bias", C.c_void_p), ("c_init", C.c_void_p)]
 
 
+class DecodeOp(C.Structure):
+    _fields_ = [("B", C.c_int32), ("T", C.c_int32), ("S", C.c_int32), ("grid", C.c_int32), ("pipe_min_n", C.c_int32)] + \
+               [(n, C.c_void_p) for n in ("slot_of_b", "enc_proj", "h", "c", "dec_proj", "par", "prev_token", "cand_valid", "tokens",
+                                          "frames", "counts", "logits")] + \
+               [("n_logits", C.c_int32), ("grid_used", C.c_int32), ("guard_bad", C.c_longlong)]
+
+
 class ModelInfo(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ("n_mels", "d_model", "n_heads", "d_head", "d_ff", "n_layers", "kernel_size", "vocab_size",
                                          "decoder_dim", "joint_dim", "n_tensors", "weight_type")] + [("vocab", C.c_char * (1025 * 8))]
@@ -59,7 +66,7 @@ EXPORTS = ["nsb_gguf_probe", "nsb_gguf_read_tensor", "nsb_default_config", "nsb_
            "nsb_stream_open", "nsb_stream_close", "nsb_stream_reset", "nsb_stream_push_pcm", "nsb_push_pcm_batch", "nsb_pop_tokens_batch", "nsb_stream_ready", "nsb_engine_step", "nsb_engine_step_begin", "nsb_engine_step_end",
            "nsb_engine_drain", "nsb_stream_pop_tokens", "nsb_stream_chunks", "nsb_detokenize", "nsb_engine_get_stats",
            "nsb_bench_prepare", "nsb_bench_step", "nsb_bench_steps", "nsb_bench_profile", "nsb_profiler_range", "nsb_bench_gemm", "nsb_trace_enable", "nsb_trace_fetch", "nsb_debug_enable", "nsb_debug_get", "nsb_debug_get_cache", "nsb_op_logmel",
-           "nsb_op_gemm", "nsb_op_gemm_ex", "nsb_op_layernorm", "nsb_transcribe_full", "nsb_stream_export", "nsb_stream_import"]
+           "nsb_op_gemm", "nsb_op_gemm_ex", "nsb_op_decode", "nsb_op_layernorm", "nsb_transcribe_full", "nsb_stream_export", "nsb_stream_import"]
 
 
 def build(force: bool = False) -> str:
@@ -120,6 +127,7 @@ def lib():
         L.nsb_op_logmel.argtypes = [vp, _i16p, ci, ci, _f32p, C.c_size_t]
         L.nsb_op_gemm.argtypes = [vp, C.c_char_p, _f32p, ci, _f32p, C.c_size_t]
         L.nsb_op_gemm_ex.argtypes = [vp, C.POINTER(GemmOp), _f32p, vp, C.c_size_t, C.POINTER(C.c_longlong)]
+        L.nsb_op_decode.argtypes = [vp, C.POINTER(DecodeOp)]
         L.nsb_op_layernorm.argtypes = [vp, _f32p, ci, vp, ci, C.c_float, _f32p, _f32p, vp, vp, ci, ci, _f32p, vp]
         L.nsb_transcribe_full.argtypes = [vp, _i16p, ci, _i32p, _i32p, ci, C.POINTER(C.c_int), C.c_void_p, C.c_size_t]
         _lib = L
@@ -364,6 +372,35 @@ class Engine:
         n = _check(lib().nsb_op_gemm_ex(self.h, C.byref(op), x, y.ctypes.data_as(C.c_void_p), y.nbytes, C.byref(bad)))
         y = y.reshape(-1)[: int(np.prod(shape[:-1])) * n].reshape(shape[:-1] + (n,)).copy()
         return y, bad.value
+
+    def op_decode(self, enc_proj: np.ndarray, h: np.ndarray, c: np.ndarray, dec_proj: np.ndarray, par, prev_token, cand_valid,
+                  slot_of_b, *, grid: int = 0, pipe_min_n: int = 0, logits: bool = True) -> dict:
+        """The step's greedy-decode launch as an operator (nsb_op_decode, include/nsb200.h). enc_proj [B, T, 640]; decoder state of
+        S slots: h, c [S, 2, 1280], dec_proj [S, 640], par / prev_token / cand_valid [S]; slot_of_b [B]. The inputs are not modified.
+        -> dict of tokens, frames [B, 10 T], counts [B], the final state (h, c, dec_proj, par, prev_token, cand_valid), logits of
+        batch row 0 [evaluations, 1025] (or None), grid_used, guard_bad."""
+        enc = np.ascontiguousarray(enc_proj, dtype=np.float32)
+        B, T = enc.shape[0], enc.shape[1]
+        f32 = lambda a: np.array(a, dtype=np.float32, order="C", copy=True)
+        i32 = lambda a: np.array(a, dtype=np.int32, order="C", copy=True)
+        out = {"h": f32(h), "c": f32(c), "dec_proj": f32(dec_proj), "par": i32(par), "prev_token": i32(prev_token),
+               "cand_valid": i32(cand_valid)}
+        S = out["par"].shape[0]
+        slots = i32(slot_of_b)
+        assert enc.shape == (B, T, 640) and slots.shape == (B,), "enc_proj [B, T, 640], slot_of_b [B]"
+        assert out["h"].size == out["c"].size == S * 2560 and out["dec_proj"].size == S * 640, "h, c [S, 2, 1280], dec_proj [S, 640]"
+        assert out["prev_token"].shape == out["cand_valid"].shape == (S,)
+        out["tokens"] = np.full((B, 10 * T), -1, dtype=np.int32)
+        out["frames"] = np.full((B, 10 * T), -1, dtype=np.int32)
+        out["counts"] = np.full(B, -1, dtype=np.int32)
+        tap = np.full((11 * T, 1025), np.nan, dtype=np.float32) if logits else None
+        p = lambda a: None if a is None else a.ctypes.data_as(C.c_void_p)
+        op = DecodeOp(B, T, S, grid, pipe_min_n, p(slots), p(enc), p(out["h"]), p(out["c"]), p(out["dec_proj"]), p(out["par"]),
+                      p(out["prev_token"]), p(out["cand_valid"]), p(out["tokens"]), p(out["frames"]), p(out["counts"]), p(tap), 0, 0, -1)
+        _check(lib().nsb_op_decode(self.h, C.byref(op)))
+        out["logits"] = tap[:min(op.n_logits, 11 * T)].copy() if logits else None
+        out["n_logits"], out["grid_used"], out["guard_bad"] = op.n_logits, op.grid_used, op.guard_bad
+        return out
 
     def op_layernorm(self, x: np.ndarray, g1, b1, *, planes=None, alpha: float = 1.0, fused: bool = False, g2=None, b2=None,
                      out_type: int = OUT_F32):

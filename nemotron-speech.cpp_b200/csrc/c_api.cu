@@ -174,6 +174,9 @@ int nsb_op_gemm(nsb_engine* e, const char* name, const float* x, int rows, float
 int nsb_op_gemm_ex(nsb_engine* e, const nsb_gemm_op* op, const float* x, void* y, size_t y_bytes, long long* guard_bad) {
     if (!e || !op || !op->weight || !x || !y) return fail(NSB_ERR_ARG, "bad argument");
     NSB_TRY return (int)e->impl->op_gemm_ex(*op, x, y, y_bytes, guard_bad); NSB_CATCH }
+int nsb_op_decode(nsb_engine* e, nsb_decode_op* op) {
+    if (!e || !op) return fail(NSB_ERR_ARG, "bad argument");
+    NSB_TRY e->impl->op_decode(*op); return NSB_OK; NSB_CATCH }
 int nsb_op_layernorm(nsb_engine* e, const float* x, int rows, const float* planes, int n_planes, float alpha, const float* g1, const float* b1,
                      const float* g2, const float* b2, int fused, int out_type, float* x_out, void* y) {
     if (!e || !x || !x_out || !y) return fail(NSB_ERR_ARG, "bad argument");

@@ -14,6 +14,7 @@
 #include <cstddef>
 #include <cstdlib>
 #include <cstring>
+#include <limits>
 
 namespace nsb {
 
@@ -1647,6 +1648,83 @@ void Engine::op_layernorm(const float* xh, int rows, const float* planes, int n_
     NSB_CUDA(cudaStreamSynchronize(st_));
     NSB_CUDA(cudaMemcpy(x_out, dx.p, n * 4, cudaMemcpyDeviceToHost));
     if (y && (!fused || g2)) NSB_CUDA(cudaMemcpy(y, dy.p, dy.bytes, cudaMemcpyDeviceToHost));
+}
+
+// The step's decode launch (run_decode_kernels / transcribe_full) on the engine's decoder weights, with state, sync buffer and outputs
+// of its own. Token and frame buffers are preset to -1 and followed by DEC_GUARD entries holding a pattern the kernel never writes.
+void Engine::op_decode(nsb_decode_op& op) {
+    constexpr int DEC_GUARD = 4096, MAX_S = 8192;
+    constexpr int32_t GUARD_VAL = 0x7FDA7FDA;
+    auto bad = [](const std::string& m) { throw std::invalid_argument("op_decode: " + m); };
+    const int B = op.B, T = op.T, S = op.S;
+    if (B < 1 || B > 1024) bad("B must be 1..1024");
+    if (T < 1 || (long long)MAX_SYMBOLS * T > 32767) bad("T must be 1..3276 (the kernel counts emissions in 16 bits)");
+    if (S < B || S > MAX_S) bad("S must be B..8192");
+    if (!op.slot_of_b || !op.enc_proj || !op.h || !op.c || !op.dec_proj || !op.par || !op.prev_token || !op.cand_valid || !op.tokens ||
+        !op.frames || !op.counts) bad("null array");
+    NSB_CUDA(cudaSetDevice(device_));
+    int sms = 0;
+    NSB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device_));
+    if (op.grid != 0 && (op.grid < 2 || op.grid % 2 != 0 || op.grid >= sms)) bad("grid must be 0 or even, 2 <= grid < SM count");
+    if (op.pipe_min_n < 0) bad("pipe_min_n must be >= 0");
+    std::vector<char> used((size_t)S, 0);
+    for (int b = 0; b < B; ++b) {
+        const int s = op.slot_of_b[b];
+        if (s < 0 || s >= S || used[s]) bad("slot_of_b must hold distinct slots in 0..S-1");
+        used[s] = 1;
+    }
+    for (int s = 0; s < S; ++s) {
+        if (op.prev_token[s] < 0 || op.prev_token[s] > BLANK) bad("prev_token must be 0..1024");
+        if (op.par[s] != 0 && op.par[s] != 1) bad("par must be 0 or 1");
+        if (op.cand_valid[s] != 0 && op.cand_valid[s] != 1) bad("cand_valid must be 0 or 1");
+    }
+
+    const size_t n_out = (size_t)B * MAX_SYMBOLS * T, n_tap = (size_t)(MAX_SYMBOLS + 1) * T * VOCAB;
+    const size_t st_f = (size_t)S * 4 * HID;
+    auto up = [](DevBuf& d, const void* h, size_t bytes) { d.alloc(bytes, false); h2d_sync(d.p, h, bytes); };
+    DevBuf d_slot, d_enc, d_h, d_c, d_proj, d_par, d_prev, d_cand, d_tok, d_frm, d_cnt, d_tap, d_tap_n, d_sync;
+    up(d_slot, op.slot_of_b, (size_t)B * 4); up(d_enc, op.enc_proj, (size_t)B * T * JOINT * 4);
+    up(d_h, op.h, st_f * 4); up(d_c, op.c, st_f * 4); up(d_proj, op.dec_proj, (size_t)S * JOINT * 4);
+    up(d_par, op.par, (size_t)S * 4); up(d_prev, op.prev_token, (size_t)S * 4); up(d_cand, op.cand_valid, (size_t)S * 4);
+    std::vector<int32_t> preset(n_out + DEC_GUARD, -1);
+    std::fill(preset.begin() + n_out, preset.end(), GUARD_VAL);
+    up(d_tok, preset.data(), preset.size() * 4); up(d_frm, preset.data(), preset.size() * 4);
+    d_cnt.alloc((size_t)B * 4, false); d_tap_n.alloc(4, false); d_sync.alloc(decode_sync_bytes(B), false);
+    if (op.logits) {
+        const std::vector<float> nan(n_tap, std::numeric_limits<float>::quiet_NaN());
+        up(d_tap, nan.data(), n_tap * 4);
+    }
+
+    DecodeArgs d{};
+    d.w.embed = embed_.as<float>();
+    for (int l = 0; l < 2; ++l) { d.w.w_ih[l] = lstm_w_[2 * l].as<float>(); d.w.w_hh[l] = lstm_w_[2 * l + 1].as<float>();
+                                  d.w.b_ih[l] = lstm_b_[2 * l].as<float>(); d.w.b_hh[l] = lstm_b_[2 * l + 1].as<float>(); }
+    d.w.pred_w = pred_w_.as<float>(); d.w.pred_b = pred_b_.as<float>(); d.w.out_w = jout_w_.as<float>(); d.w.out_b = jout_b_.as<float>();
+    d.s.hbuf = d_h.as<float>(); d.s.cbuf = d_c.as<float>(); d.s.par = d_par.as<int>();
+    d.s.dec_proj = d_proj.as<float>(); d.s.prev_token = d_prev.as<int>(); d.s.cand_valid = d_cand.as<int>();
+    d.enc_proj = d_enc.as<float>(); d.slot_of_b = d_slot.as<int>(); d.B = B; d.T = T;
+    d.out_tokens = d_tok.as<int>(); d.out_count = d_cnt.as<int>(); d.out_frames = d_frm.as<int>();
+    d.logits_tap = op.logits ? d_tap.as<float>() : nullptr; d.logits_tap_cap = op.logits ? (MAX_SYMBOLS + 1) * T : 0;
+    d.logits_tap_n = d_tap_n.as<int>();
+    const int used_grid = launch_decode(d, d_sync.p, st_, op.grid, op.pipe_min_n);
+    NSB_CUDA(cudaStreamSynchronize(st_));
+
+    auto down = [](void* h, const DevBuf& dv, size_t bytes) { NSB_CUDA(cudaMemcpy(h, dv.p, bytes, cudaMemcpyDeviceToHost)); };
+    long long nbad = 0;
+    for (const DevBuf* o : {&d_tok, &d_frm}) {
+        down(preset.data(), *o, preset.size() * 4);
+        for (size_t i = n_out; i < preset.size(); ++i) nbad += preset[i] != GUARD_VAL;
+        memcpy(o == &d_tok ? op.tokens : op.frames, preset.data(), n_out * 4);
+    }
+    down(op.counts, d_cnt, (size_t)B * 4);
+    down(op.h, d_h, st_f * 4); down(op.c, d_c, st_f * 4); down(op.dec_proj, d_proj, (size_t)S * JOINT * 4);
+    down(op.par, d_par, (size_t)S * 4); down(op.prev_token, d_prev, (size_t)S * 4); down(op.cand_valid, d_cand, (size_t)S * 4);
+    int ne = 0;
+    down(&ne, d_tap_n, 4);
+    op.n_logits = ne;
+    if (op.logits) down(op.logits, d_tap, (size_t)std::min(ne, (MAX_SYMBOLS + 1) * T) * VOCAB * 4);
+    op.grid_used = used_grid;
+    op.guard_bad = nbad;
 }
 
 }  // namespace nsb

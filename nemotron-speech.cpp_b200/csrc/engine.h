@@ -105,6 +105,7 @@ public:
     long long op_logmel(const int16_t* pcm, int n_streams, int n_samples, float* out, size_t cap);
     long long op_gemm(const std::string& name, const float* x, int rows, float* y, size_t cap);
     long long op_gemm_ex(const nsb_gemm_op& op, const float* x, void* y, size_t y_bytes, long long* guard_bad);
+    void op_decode(nsb_decode_op& op);
     void op_layernorm(const float* x, int rows, const float* planes, int n_planes, float alpha, const float* g1, const float* b1,
                       const float* g2, const float* b2, bool fused, int out_type, float* x_out, void* y);
     // Non-streaming batch path (nemo_encode, reference src/nemo-ggml.cpp:1467-1535) for one utterance: whole-utterance log-mel ->

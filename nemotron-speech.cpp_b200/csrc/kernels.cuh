@@ -139,8 +139,9 @@ struct DecodeArgs {
     float* logits_tap; int logits_tap_cap; int* logits_tap_n;   // optional: logits of batch row 0 per evaluation
 };
 // persistent kernel; sync_buf holds decode_sync_bytes(B) bytes. narrow_ctas = 0: one CTA per SM (cooperative launch); > 0: that many CTAs
-// as CTA pairs, sharing the GPU with other kernels (decode overlap). Returns the grid size used
-int launch_decode(const DecodeArgs& a, void* sync_buf, cudaStream_t st, int narrow_ctas = 0);
+// as CTA pairs, sharing the GPU with other kernels (decode overlap). pipe_min_n > 0 replaces the default streams-per-phase threshold of
+// the pipelined tiles on a wide grid (operator tests). Returns the grid size used
+int launch_decode(const DecodeArgs& a, void* sync_buf, cudaStream_t st, int narrow_ctas = 0, int pipe_min_n = 0);
 int decode_narrow_ctas();          // NSB_DECODE_CTAS, default 20 (148 SMs - the 128 CTAs of the widest small-batch encoder kernel)
 size_t decode_sync_bytes(int B);
 

@@ -663,13 +663,13 @@ int decode_narrow_ctas() {
 // CTA pairs (clusters of 2: a pair takes one TPC, so the CTA-pair GEMMs of a concurrently running encoder keep their TPCs whole) with a
 // plain launch: the kernel then shares the GPU with the next step's encoder. Its grid barrier needs every CTA resident at some
 // point, which a grid this small reaches as soon as a few SMs are free -- nothing the other kernels run ever waits on this one.
-int launch_decode(const DecodeArgs& a_in, void* sync_buf, cudaStream_t st, int narrow_ctas) {
+int launch_decode(const DecodeArgs& a_in, void* sync_buf, cudaStream_t st, int narrow_ctas, int pipe_min_n) {
     const int full = decode_grid();
     if (a_in.B > MAXB) throw CudaError("decode: more than 1024 streams in one step");
     DecodeArgs a = a_in;
     // full-width grid: pipelined tiles from this many streams per phase on (below, one or two one-shot items per CTA are as good or better)
     static const int pipe_n = [] { const char* e = getenv("NSB_DECODE_PIPE_N"); return e ? atoi(e) : 65; }();
-    a.pipe_min_n = pipe_n;
+    a.pipe_min_n = pipe_min_n > 0 ? pipe_min_n : pipe_n;
     a.barrier = reinterpret_cast<unsigned*>(sync_buf);
     a.best = reinterpret_cast<unsigned long long*>((char*)sync_buf + 16);
     NSB_CUDA(cudaMemsetAsync(sync_buf, 0, decode_sync_bytes(a.B), st));           // barrier counter + argmax keys
